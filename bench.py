@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm  (torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...   # CPU arm: the oracle port on host cores
+    python bench.py ... --dump-outputs DIR                    # also write a seeded sample of the pool after the timed steps
 
 Workload (config.workload): Llama-3-8B bf16, 291 tensors / 4 safetensors shards / 16,060,522,496 B, synthetic
 content, files warm in tmpfs/page cache.  A "step" = one pass of the hot path over the whole checkpoint:
@@ -37,6 +38,7 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -51,8 +53,11 @@ UNIT = "GB/s"
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of every timed loop (kernel stage, e2e, CPU baseline, secondary records)")
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what the last one made resident (rank 0's pool, tensor by tensor as its manifest describes it) "
+                         "to DIR/<tensor name>.npy, a seeded sample of large tensors, at most 64 MB in all (see dump_outputs)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="llama3-8b", choices=["llama3-8b", "mixtral-q4k", "gpt2", "llama3-70b-scatter"])
     ap.add_argument("--qtype", default="Q4_K", help="mixtral-q4k: block type of the weights (Q4_K = the BASELINE config; Q4_0, Q5_K, IQ4_XS, ... "
@@ -81,6 +86,8 @@ def parse():
                     help="broadcast order: fused convert+fan-out by P2P stores (p2p), all-gather the file bytes then convert locally (raw), or convert into own "
                          "pool + slice buffer and pull the peers' slices (pull: peers map 1/N of the bytes).  auto = p2p (measured best on every count at N = 8)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the GPU pool; the CPU arm (--impl reference) has none")
     if a.fanout == "auto":
         # Measured at N = 8 (profiles/README.md, round 2): with pools in 2 MiB multiples the seven 16 GB pool mappings of the P2P-store order take
         # 0.05-0.07 s (3.6 s in round 1), so it has the shorter time-to-ready, the faster kernel stage (20.0 vs 25.2 ms) and the faster e2e step
@@ -336,6 +343,47 @@ def emit(line: dict) -> None:
     else:
         sys.stdout.write(data.decode())
         sys.stdout.flush()
+
+
+DUMP_BYTES = 48 << 20  # --dump-outputs: values written for all tensors together (the files, .npy headers included, stay under 64 MB)
+DUMP_RUN = 4096        # elements per sampled run of a large tensor
+# pool dtype -> (element type as stored, type written); FP8, sub-byte and block-quantised types are written as their bytes, one value per byte
+_DUMP_TYPES = {"BF16": (np.uint16, np.float32), "F16": (np.float16, np.float32), "F32": (np.float32, np.float32), "F64": (np.float64, np.float64),
+               **{k: (v, np.float64) for k, v in (("BOOL", np.uint8), ("U8", np.uint8), ("I8", np.int8), ("U16", np.uint16), ("I16", np.int16),
+                                                  ("U32", np.uint32), ("I32", np.int32), ("U64", np.uint64), ("I64", np.int64))}}
+_DUMP_BYTEWISE = (np.uint8, np.float32)
+
+
+def _dump_values(raw: np.ndarray, dtype: str) -> np.ndarray:
+    src, dst = _DUMP_TYPES.get(dtype, _DUMP_BYTEWISE)
+    v = raw.view(src)
+    if dtype == "BF16":
+        return (v.astype(np.uint32) << 16).view(np.float32)
+    return v.astype(dst)
+
+
+def dump_outputs(out_dir: str, tensors, read) -> None:
+    """--dump-outputs: what a caller of the timed path receives — every tensor of the pool, as the manifest describes it — written as
+    out_dir/<tensor name>.npy.  `read(offset, nbytes)` returns pool bytes.  A tensor whose values fit its share of DUMP_BYTES is written whole in
+    its shape; a larger one as the 1-D concatenation of runs of DUMP_RUN elements drawn with a seed taken from its name, so that the same
+    arguments select the same elements in every run and two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // max(len(tensors), 1)
+    for t in tensors:
+        src, dst = _DUMP_TYPES.get(t["dtype"], _DUMP_BYTEWISE)
+        isz = np.dtype(src).itemsize
+        n, per = t["nbytes"] // isz, share // np.dtype(dst).itemsize
+        if n <= per:
+            vals = _dump_values(read(t["offset"], n * isz), t["dtype"])
+            if n == int(np.prod(t["shape"])):
+                vals = vals.reshape(t["shape"])
+        else:
+            run = min(DUMP_RUN, per)
+            rng = np.random.default_rng(zlib.crc32(t["name"].encode()))
+            starts = np.sort(rng.choice(n // run, per // run, replace=False)) * run
+            vals = np.concatenate([_dump_values(read(t["offset"] + int(s) * isz, run * isz), t["dtype"]) for s in starts])
+        with open(os.path.join(out_dir, t["name"].replace(os.sep, "_") + ".npy"), "wb") as f:
+            np.save(f, vals)
 
 
 def main():
@@ -612,6 +660,8 @@ def main():
                 "read_mode": os.environ.get("KUKEON_GPULOAD_READ", "auto"), "e2e_ms_each": [t * 1e3 for t in e2e_ts], "steps_detail": step_detail[-args.steps:],
                 "config": {"readers": args.readers, "slots": args.slots, "slot_mb": args.slot_mb, "zerocopy": args.zerocopy, "numa_pin": not args.no_numa_pin,
                            "chunks_per_load": chunks_per_load, "kk_open_s": t_open}}
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, m.manifest(local)["tensors"], lambda off, n: m.read(local, off, n))
         m.release()
         pool.close()
         barrier()
@@ -655,6 +705,8 @@ def main():
     wall = time.perf_counter() - wall0
     tc1 = time.time()
     ck = clocks.stop(tc0, tc1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, m.manifest(local)["tensors"], lambda off, n: m.read(local, off, n))
     dev_ms = allmax(sum(step_ms))
     value = delivered * args.steps / (dev_ms / 1e3) / 1e9
     n_launch = len(launch_ms[0])
@@ -754,7 +806,7 @@ def main():
             ctx = cpu_port_setup(path, None if file_bytes <= (40 << 30) else 40 << 30)
             cpu_port_step(ctx)  # untimed: parallel first touch of the output buffer
             cpu_port_step(ctx)
-            ts = [cpu_port_step(ctx) for _ in range(5)]
+            ts = [cpu_port_step(ctx) for _ in range(args.steps)]
             cpu = {"value": ctx[3] / statistics.median(ts) / 1e9, "unit": UNIT, "cores": os.cpu_count() or 1, "kind": "port",
                    "sample": (("the whole checkpoint" if ctx[3] == file_bytes else f"first {ctx[3] / 1e9:.2f} GB of the checkpoint") +
                               f" ({ctx[3] / 1e9:.2f} GB), median of {len(ts)} passes after 2 untimed ones, pread + convert into host memory, all OpenMP threads"),
@@ -907,7 +959,7 @@ def secondary_kernel_stage(args, pool, gpupool, modelhub, peak, write_peak, work
             m.stage_resident()
             for _ in range(3):
                 m.convert_resident()
-            steps = 10
+            steps = args.steps
             runs = [m.convert_resident() for _ in range(steps)]
             part = m.stats()["parts"][0]
         finally:

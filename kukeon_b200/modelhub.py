@@ -229,6 +229,21 @@ def forget_pool(model) -> None:
         del _POOL_SUMS[k]
 
 
+_SUN_PATH_MAX = 107  # sockaddr_un.sun_path: 108 bytes including the terminating NUL
+
+
+def _at_unix_path(op, path: str):
+    """`op(address)` — a socket's bind or connect — for the Unix socket at `path`.  A cell's metadata directory can be deeper than sun_path
+    allows; a longer path is reached as /proc/self/fd/<directory fd>/<name>, which the kernel resolves to the same file."""
+    if len(os.fsencode(path)) <= _SUN_PATH_MAX:
+        return op(path)
+    dfd = os.open(os.path.dirname(path) or ".", os.O_PATH | os.O_DIRECTORY)
+    try:
+        return op(f"/proc/self/fd/{dfd}/{os.path.basename(path)}")
+    finally:
+        os.close(dfd)
+
+
 class PoolFdServer(threading.Thread):
     """Hands the file descriptor of a VMM pool to whoever connects to `path` (a Unix socket staged in the directory that is bind-mounted
     read-only into the agent container — like a docker.sock, the socket stays connectable through the mount).  One message per connection:
@@ -244,7 +259,7 @@ class PoolFdServer(threading.Thread):
         except FileNotFoundError:
             pass
         self.sock = socket.socket(socket.AF_UNIX, socket.SOCK_STREAM)
-        self.sock.bind(path)
+        _at_unix_path(self.sock.bind, path)
         os.chmod(path, 0o660)
         self.sock.listen(16)
         self.sock.settimeout(0.2)
@@ -293,7 +308,7 @@ def unmount(spec: MountSpec) -> None:
 def receive_pool_fd(sock_path: str) -> tuple:
     """Agent side: connect to the staged socket, returns (fd, mapped_bytes).  The caller maps it with gpupool.ImportedPool and closes the fd."""
     with socket.socket(socket.AF_UNIX, socket.SOCK_STREAM) as c:
-        c.connect(sock_path)
+        _at_unix_path(c.connect, sock_path)
         msg, fds, _, _ = socket.recv_fds(c, 8, 1)
         if len(msg) != 8 or len(fds) != 1:
             raise OSError("pool fd server sent no descriptor")

@@ -62,6 +62,38 @@ def test_reference_arm_prints_one_json_line(tmp_path):
     assert d["config"]["same_config"] is True and "whole checkpoint" in d["cpu_baseline"]["sample"]
 
 
+def test_dump_outputs_writes_every_pool_tensor_and_samples_large_ones_by_seed(tmp_path, monkeypatch):
+    """bench.dump_outputs (--dump-outputs) over an oracle pool: a tensor that fits its share comes out whole, in its shape, value for value;
+    a larger one as runs of DUMP_RUN consecutive elements of the tensor; a second dump is identical; the files stay within the budget."""
+    import numpy as np
+
+    from oracle import oracle
+    from tests import helpers
+    p = str(tmp_path / "m.safetensors")
+    helpers.mixed_safetensors(p)
+    shards, recs = oracle.index_path(p)
+    pool, plan = oracle.expected_pool(shards, recs)
+    tensors = [dict(name=t["name"], dtype=t["dtype"], shape=t["shape"], offset=t["pool_offset"], nbytes=t["nbytes"]) for t in plan]
+    monkeypatch.setattr(bench, "DUMP_BYTES", 512 << 10)  # h.bf16.big (716,800 values) is sampled, the rest fits
+    monkeypatch.setattr(bench, "DUMP_RUN", 256)
+    for k in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / k), tensors, lambda off, n: pool[off:off + n].copy())
+    assert sorted(os.listdir(tmp_path / "a")) == sorted(t["name"] + ".npy" for t in tensors)
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= (512 << 10) + 128 * len(tensors)
+    for t in tensors:
+        a, b = np.load(tmp_path / "a" / (t["name"] + ".npy")), np.load(tmp_path / "b" / (t["name"] + ".npy"))
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b, equal_nan=True)
+        raw = pool[t["offset"]:t["offset"] + t["nbytes"]]
+        full = {"BF16": lambda: (raw.view(np.uint16).astype(np.uint32) << 16).view(np.float32), "F32": lambda: raw.view(np.float32),
+                "I64": lambda: raw.view(np.int64).astype(np.float64), "U8": lambda: raw.astype(np.float64), "BOOL": lambda: raw.astype(np.float64)}[t["dtype"]]()
+        if t["name"] == "h.bf16.big":
+            runs = full.reshape(-1, 256)
+            assert a.ndim == 1 and a.size and a.size % 256 == 0 and a.size < full.size
+            assert all(any(np.array_equal(r, q, equal_nan=True) for q in runs) for r in a.reshape(-1, 256))
+        else:
+            assert a.shape == tuple(t["shape"]) and np.array_equal(a.reshape(-1), full, equal_nan=True)
+
+
 def test_pending_gpu_scripts_point_at_things_that_exist():
     """The GPU command files still to be spent (tools/r02/*.sh; spent ones move to tools/history/) each cost box minutes: they must parse and
     every script they run must exist and parse."""

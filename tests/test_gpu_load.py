@@ -304,10 +304,13 @@ def test_mount_exports_manifest_and_ipc_handle_to_another_process(pool, tmp_path
         env = dict(e.split("=", 1) for e in spec.env)
         assert env["KUKEON_GPUPOOL_DEVICE_UUID"] == ident["uuid"] == man["deviceUUID"] and ident["uuid"].startswith("GPU-") and len(ident["uuid"]) == 40
         assert env["KUKEON_GPUPOOL_PCI_BUS_ID"] == ident["pci_bus_id"] == man["pciBusId"]
-        if os.path.isdir(modelhub.NVIDIA_PROC_GPUS):  # device node from the driver's table, not from the ordinal
+        if os.path.exists(os.path.join(modelhub.NVIDIA_PROC_GPUS, ident["pci_bus_id"], "information")):  # device node from the driver's table, not from the ordinal
             minor = modelhub.device_minor(ident["pci_bus_id"])
             wd = modelhub.Mount(m, 0, str(tmp_path / "cell" / "container2"), with_devices=True)
             assert f"/dev/nvidia{minor}" in [d["path"] for d in wd.devices] and "/dev/nvidiactl" in [d["path"] for d in wd.devices]
+        else:  # a container can mask the driver's table (the directory present, this GPU's entry absent): no node is guessed then
+            with pytest.raises(FileNotFoundError):
+                modelhub.Mount(m, 0, str(tmp_path / "cell" / "container2"), with_devices=True)
         assert os.path.getsize(os.path.join(spec.host_dir, "ipc.handle")) == 64
         t = want[7]  # h.bf16.big
         r = subprocess.run([sys.executable, "-c", _CHILD, os.path.join(spec.host_dir, "ipc.handle"), str(t["pool_offset"]), "4096", ident["uuid"]],

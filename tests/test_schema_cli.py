@@ -153,6 +153,42 @@ class _StubModel:
                                         "pciBusId": f"0000:{0x1b + device:02x}:00.0", "tensors": [{"name": f"w{self.tag}"}]}
 
 
+class _StubVmmModel:
+    """A VMM pool as Mount sees it: export_fd(device) -> (fd, mapped bytes) and manifest(device); the fd is that of a plain file."""
+
+    def __init__(self, path):
+        self.path = path
+
+    def export_fd(self, device):
+        return os.open(self.path, os.O_RDONLY), os.path.getsize(self.path)
+
+    def manifest(self, device):
+        return {"apiVersion": "kukeon.gpupool/v1", "device": device, "deviceUUID": "GPU-00000000-aaaa-bbbb-cccc-dddddddddddd", "pciBusId": "0000:1b:00.0",
+                "tensors": []}
+
+
+def test_vmm_mount_serves_the_pool_fd_from_a_directory_deeper_than_sun_path(tmp_path):
+    """The staged pool.sock lives in the cell's metadata directory, whatever its depth: a socket path longer than sockaddr_un allows is still
+    bound by Mount and reached by receive_pool_fd."""
+    from kukeon_b200 import modelhub
+    pool_file = tmp_path / "pool.bin"
+    pool_file.write_bytes(bytes(range(256)) * 16)
+    cdir = str(tmp_path / ("realm-" + "r" * 40) / ("cell-" + "c" * 40) / "container")
+    spec = modelhub.Mount(_StubVmmModel(str(pool_file)), 0, cdir)
+    try:
+        sock = os.path.join(spec.host_dir, "pool.sock")
+        assert len(sock) > 108 and os.path.exists(sock)
+        assert "KUKEON_GPUPOOL_FD_SOCKET=/run/kukeon/gpupool/pool.sock" in spec.env
+        fd, size = modelhub.receive_pool_fd(sock)
+        try:
+            assert size == 4096 and os.pread(fd, 4096, 0) == pool_file.read_bytes()
+        finally:
+            os.close(fd)
+    finally:
+        modelhub.unmount(spec)
+    assert not os.path.exists(sock)
+
+
 def test_mount_single_and_named_models(tmp_path):
     from kukeon_b200 import modelhub
     cdir = str(tmp_path / "cell" / "work")
